@@ -19,6 +19,8 @@ A step = one complete aggregation of the batch: Partial -> (murmur3 pmod N excha
                 computation (per-group sums / counts, group ownership disjoint across ranks); a mismatch exits non-zero
 
 `--impl reference` times the CPU restatement alone on the same M2 workload (the Rust reference cannot be built here).
+`--dump-outputs DIR` writes the headline's last timed result as DIR/k1.npy, k2.npy, sum_v.npy (float64, rows in key order);
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                     # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "rows/sec on TPC-DS q1 hash-agg+filter at 1/2/4/8 B200; HBM GB/s vs 8 TB/s"
 CARD = 1 << 20
@@ -519,6 +522,8 @@ def run_ours(args):
     if not ok:
         failures.append("M2")
     verified = {"M2": dict(ok=ok, **info)}
+    if args.dump_outputs:
+        dump_m2_outputs(torch, dist, r2, args.dump_outputs)
 
     # ---- e2e: host buffers through the C ABI (M2) -------------------------------------------------------------------
     import numpy as np
@@ -615,6 +620,26 @@ def run_ours(args):
     if failures:
         sys.stderr.write(f"bench.py: RESULT VERIFICATION FAILED for {failures}\n")
         sys.exit(3)
+
+
+def dump_m2_outputs(torch, dist, runner, out_dir):
+    """The M2 result of the last timed step, the columns k1, k2, sum_v the Final stage returns, merged over the ranks and
+    saved as out_dir/<column>.npy.  A hash aggregate emits its groups in no fixed order, so the rows are put in key order
+    (k1 * 8 + k2) to make two runs comparable row for row; float64 holds every value exactly (|sum_v| < 2^53)."""
+    import numpy as np
+    sums = torch.zeros(CARD, dtype=torch.int64, device=runner.dev)
+    seen = torch.zeros(CARD, dtype=torch.int64, device=runner.dev)
+    for cols in (device_cols(d, torch) for d in runner.last or []):
+        gi = cols[0] * K2_CARD + cols[1]
+        sums.index_add_(0, gi, cols[2]); seen.index_add_(0, gi, torch.ones_like(gi))
+    if runner.world > 1:
+        dist.all_reduce(sums); dist.all_reduce(seen)
+    if runner.rank != 0:
+        return
+    gi = torch.nonzero(seen).squeeze(1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("k1", gi // K2_CARD), ("k2", gi % K2_CARD), ("sum_v", sums[gi])):
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 def mem_available_bytes():
@@ -729,7 +754,12 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's last timed result to DIR/<column>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

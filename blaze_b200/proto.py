@@ -4,8 +4,8 @@ field numbers, so bytes produced here are byte-compatible with what the Spark si
 what `auron-serde` decodes (native-engine/auron-serde/proto/auron.proto:27-55, 58-125, 143-148,
 169-198, 271-311, 363-366, 470-473, 489-510, 675-696, 729-740, 751-760, 786-789, 824-826, 860-896).
 
-`tests/test_proto_compat.py` re-parses the reference .proto text (when /root/reference is
-mounted) and checks every field number declared here against it.
+`tests/test_proto_compat.py` checks every field number declared here against the reference's
+field table, stored in `tests/golden/auron_proto_fields.json`.
 """
 from __future__ import annotations
 

@@ -1,38 +1,21 @@
 """blaze_b200/proto.py declares the hot-path subset of the reference's auron.proto programmatically;
-when the reference is mounted, every message/field/number/type is checked against the .proto text."""
+every message/field/number/type is checked against the reference's field table, stored in
+tests/golden/auron_proto_fields.json (regenerated from the .proto text by tests/golden/make_proto_fields.py)."""
+import json
 import os
-import re
-
-import pytest
 
 from blaze_b200 import proto as P
 
-REF = "/root/reference/native-engine/auron-serde/proto/auron.proto"
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "auron_proto_fields.json")
 
 
-def _parse_reference():
-    text = re.sub(r"//.*", "", open(REF).read())
-    msgs = {}
-    for m in re.finditer(r"message\s+(\w+)\s*\{", text):
-        name, i, depth = m.group(1), m.end(), 1
-        j = i
-        while depth:
-            depth += {"{": 1, "}": -1}.get(text[j], 0)
-            j += 1
-        body = text[i:j - 1]
-        fields = {}
-        for f in re.finditer(r"(repeated\s+)?([\w.]+)\s+(\w+)\s*=\s*(\d+)\s*;", body):
-            fields[f.group(3)] = (int(f.group(4)), f.group(2), bool(f.group(1)))
-        msgs[name] = fields
-    enums = {}
-    for m in re.finditer(r"enum\s+(\w+)\s*\{([^}]*)\}", text):
-        enums[m.group(1)] = {a: int(b) for a, b in re.findall(r"(\w+)\s*=\s*(\d+)\s*;", m.group(2))}
-    return msgs, enums
+def _load_reference():
+    ref = json.load(open(REF))
+    return ref["messages"], ref["enums"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference not mounted")
 def test_field_numbers_match_reference_proto():
-    msgs, enums = _parse_reference()
+    msgs, enums = _load_reference()
     from google.protobuf import descriptor_pb2 as dpb
     F = dpb.FieldDescriptorProto
     scalar = {F.TYPE_STRING: "string", F.TYPE_BYTES: "bytes", F.TYPE_BOOL: "bool", F.TYPE_UINT32: "uint32",
